@@ -16,6 +16,12 @@ One JSON line on stdout (rank 0). Keys beyond the base contract: "roofline" (tcg
 FLOP/s from CUDA events around every GEMM launch in a profiled pass of the same steps), "cpu_baseline"
 (oracle port on a bounded sample, rank 0, N=1), "e2e" (same metric through s3b_forward_host: pinned host
 waveforms in, all hidden states back to pinned host memory, copies inside the timed region), "clocks".
+
+    python bench.py ... --dump-outputs DIR
+
+also writes, from rank 0, what the last timed step returned as float32 .npy files (see dump_outputs): features.npy
+(the weighted sum, or the fbank features) and hidden_states.npy (every layer). Inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -86,6 +92,38 @@ def seeded_wav(idx: int, n: int):
 
     g = torch.Generator().manual_seed(1000 + idx)
     return torch.randn(n, generator=g)
+
+
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this many bytes in all (npy headers included)
+NPY_HEADER = 128
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write each output as out_dir/<name>.npy (float32). An output is a [B, T, D] tensor, or a sequence of them
+    written stacked as [N, B, T, D]. Each output may use an equal share of DUMP_BYTES, plus whatever the outputs before
+    it left unused. One larger than its share keeps a fixed sample of its B * T frames instead, [(N,) k, D]: the first
+    k of torch.randperm(B * T) under seed 0, in ascending order. Their flat indices b * T + t go to
+    out_dir/<name>_frames.npy (float64)."""
+    import numpy as np
+    import torch
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    left = DUMP_BYTES
+    for i, (name, x) in enumerate(outputs.items()):
+        share = left // (len(outputs) - i)
+        layers = list(x) if isinstance(x, (list, tuple)) else [x]
+        B, T, D = layers[0].shape
+        frame_bytes = len(layers) * D * 4
+        if NPY_HEADER + B * T * frame_bytes > share:
+            k = (share - 2 * NPY_HEADER) // (frame_bytes + 8)
+            idx = torch.randperm(B * T, generator=torch.Generator().manual_seed(0))[:k].sort().values
+            np.save(out / f"{name}_frames.npy", idx.double().numpy())
+            left -= (out / f"{name}_frames.npy").stat().st_size
+            layers = [h.reshape(B * T, D)[idx.to(h.device)] for h in layers]
+        arr = torch.stack([h.float().cpu() for h in layers]).numpy()
+        np.save(out / f"{name}.npy", arr if isinstance(x, (list, tuple)) else arr[0])
+        left -= (out / f"{name}.npy").stat().st_size
 
 
 class ClockSampler:
@@ -175,8 +213,8 @@ def usable_cores() -> int:
 
 def cpu_arm(cfg_key: str, n_utts: int, steps: int, warmup: int, budget_s: float = None):
     """Time the reference's CPU implementation of the step on `n_utts` utterances of the workload, all usable host
-    threads. kind = "reference": the UNMODIFIED reference (s3prl UpstreamExpert + Featurizer from /root/reference or the
-    oracle/_ref install, oracle/build_ref.py) on the fabricated checkpoint; kind = "port": the oracle restatement
+    threads. kind = "reference": the UNMODIFIED reference (s3prl UpstreamExpert + Featurizer from the checkout beside this
+    repository or S3PRL_REFERENCE, else the oracle/_ref install, oracle/build_ref.py) on the fabricated checkpoint; kind = "port": the oracle restatement
     (only when the reference is not present). Returns (frames/s, ms/step, cores, kind, steps actually timed)."""
     import torch
 
@@ -335,6 +373,8 @@ def run_fbank(args):
         "gpu_launches": 5 * args.steps,
         "clocks": clocks,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"features": out})
     if not args.no_cpu_baseline:
         fps, ms, cores, kind, timed = cpu_arm(args.config, c["batch"], 20, 2)
         line["cpu_baseline"] = {"value": fps, "unit": "frames/s", "cores": cores, "kind": kind,
@@ -389,10 +429,11 @@ def run_ours(args):
         gatherer = FeatureGatherer((per, T, D), device, mode=args.gather)
 
     def step():
-        res = expert(wavs)
+        """What a caller of the hot path receives: (hidden states, weighted-sum features)."""
+        hs = expert(wavs)["hidden_states"]
         if gatherer is not None:  # weighted sum written straight into every rank's gathered buffer (or NCCL)
-            return gatherer.weighted_sum_gather(res["hidden_states"], fw)
-        return weighted_sum(res["hidden_states"], fw)
+            return hs, gatherer.weighted_sum_gather(hs, fw)
+        return hs, weighted_sum(hs, fw)
 
     def barrier():
         if world > 1:
@@ -403,8 +444,10 @@ def run_ours(args):
         sampler = ClockSampler(local_rank) if rank == 0 else None
         if sampler:
             sampler.start()  # nvidia-smi needs ~100 ms to come up: start it before the warm-up
+        # the warm-up keeps the previous step's outputs alive as the timed loop does, so that the allocator already
+        # holds both output buffers when timing starts
         for _ in range(max(args.warmup, 3)):
-            step()
+            last = step()
         if gatherer is not None:
             gatherer.finish()
         # ---- timed region: device-resident inputs ----------------------------------------------------------
@@ -417,7 +460,7 @@ def run_ours(args):
         e0.record()
         t_host = time.perf_counter()
         for _ in range(args.steps):
-            step()
+            last = step()
         if gatherer is not None:
             gatherer.finish()  # every rank's last gathered buffer is complete (all peers' pushes have landed)
         host_enqueue_ms = (time.perf_counter() - t_host) * 1e3 / args.steps  # CPU time to enqueue one step
@@ -487,6 +530,9 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:  # rank 0: the gathered features of the whole batch, the hidden states of its own shard
+        hidden_states, features = last
+        dump_outputs(args.dump_outputs, {"features": features, "hidden_states": hidden_states})
 
     peaks = {}
     try:
@@ -565,7 +611,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--emulate-world", type=int, default=0,
                     help="development aid: time one rank's shard of an N-GPU run on one GPU (no gather); not a bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes this project's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     elif CONFIGS[args.config]["model"] == "fbank":

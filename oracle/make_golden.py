@@ -1,8 +1,8 @@
-"""TEST INFRASTRUCTURE — generates tests/golden/*.pt by EXECUTING THE REFERENCE (s3prl @ /root/reference).
+"""TEST INFRASTRUCTURE — generates tests/golden/* by EXECUTING THE REFERENCE (s3prl, see oracle/ref_runtime.py).
 
-Run in the build container only (the reference does not travel to the GPU box):
+Only where an s3prl checkout is at hand; the tests read the stored results and never need the reference:
 
-    PYTHONPATH=/root/reference python oracle/make_golden.py [--only hubert_base]
+    python oracle/make_golden.py [--only hubert_base]     # reference at ../reference, or S3PRL_REFERENCE=/path/to/s3prl
 
 For every architecture it
   1. fabricates the deterministic checkpoint (s3prl_b200.upstream.weights.fabricate_state_dict, seed 0),
@@ -62,7 +62,7 @@ def seeded_wavs(lens, seed):
     return [torch.randn(n, generator=g) for n in lens]
 
 
-from ref_runtime import reference_expert  # noqa: E402  (the reference itself on a fabricated checkpoint)
+from ref_runtime import activate, reference_expert  # noqa: E402  (the reference itself on a fabricated checkpoint)
 
 
 def make_model_fixture(name: str, fixture: str = None):
@@ -193,14 +193,126 @@ def make_spectrogram_fixture():
     torch.save(out, GOLDEN / "spectrogram.pt")
 
 
+class FakeUpstream:
+    """The static facts s3prl.nn.Featurizer reads from an upstream: n layers of width 16 at stride 320."""
+
+    def __init__(self, n):
+        self.num_layers, self.hidden_sizes, self.downsample_rates = n, [16] * n, [320] * n
+
+
+def fake_s3prl_upstream(cls):
+    """An S3PRLUpstream (the reference's class or s3prl_b200.nn's) around a fake three-layer upstream with the conv
+    stack's frame rule, built without the constructor (which would load a model)."""
+
+    class Fake(torch.nn.Module):
+        def forward(self, wavs):
+            frames = max((len(w) - 400) // 320 + 1 if len(w) >= 400 else 0 for w in wavs)
+            base = torch.arange(len(wavs) * frames * 2, dtype=torch.float32).view(len(wavs), frames, 2)
+            return {"hidden_states": [base + k for k in range(3)]}
+
+    obj = cls.__new__(cls)
+    torch.nn.Module.__init__(obj)
+    obj.upstream, obj.normalize = Fake(), False
+    obj._hidden_sizes, obj._downsample_rates = [2] * 3, [320] * 3
+    obj._num_layers = 3  # read by the reference's num_layers property
+    return obj
+
+
+# the cases of tests/test_host_cpu.py that nn_upstream.pt answers
+FEATURIZER_CASES = ((None, False), ([4, 0, 2], False), (None, True), ([1, 3], True))
+S3PRL_UPSTREAM_LENS = ([16000, 9000, 3200], [16001, 480], [700, 500], [32000, 31999], [1281, 1280, 1279], [48000])
+S3PRL_UPSTREAM_REFUSED_LENS = ([960, 961], [1000, 900])  # 2 frames from the conv rule where ceil(L / 320) = 4
+
+
+def make_nn_fixture():
+    """The reference's s3prl.nn wrappers (s3prl/nn/upstream.py:166-384) on the CPU: Featurizer outputs and weight
+    gradients (layer selection, normalize), UpstreamDownstreamModel plumbing, S3PRLUpstream length bookkeeping on a
+    fake upstream, and which inputs the latter refuses."""
+    from s3prl.nn.upstream import Featurizer, S3PRLUpstream, UpstreamDownstreamModel
+
+    g = torch.Generator().manual_seed(0)
+    hs = [torch.randn(3, 7, 16, generator=g) for _ in range(5)]
+    lens = [torch.tensor([7, 5, 2])] * 5
+    featurizer = []
+    for sel, norm in FEATURIZER_CASES:
+        f = Featurizer(FakeUpstream(5), sel, norm)
+        w = torch.randn(len(f.weights), generator=g)
+        with torch.no_grad():
+            f.weights.copy_(w)
+        h, h_len = f(hs, lens)
+        h.square().sum().backward()
+        featurizer.append({"layer_selections": list(f.layer_selections), "weights": w, "hs": h.detach(), "hs_len": h_len,
+                           "grad": f.weights.grad.clone(), "output_size": f.output_size,
+                           "downsample_rate": f.downsample_rate})
+    single = Featurizer(FakeUpstream(1))
+
+    class Up(torch.nn.Module):
+        num_layers, hidden_sizes, downsample_rates = 5, [16] * 5, [320] * 5
+
+        def forward(self, wav, wav_len):
+            return hs, lens
+
+    class Down(torch.nn.Module):
+        output_size = 3
+
+        def forward(self, h, h_len, scale=1.0):
+            return h[..., :3] * scale, h_len
+
+    udm = UpstreamDownstreamModel(Up(), Featurizer(Up()), Down())
+    udm_hs, udm_len = udm(None, None, scale=2.0)
+
+    ref, cases = fake_s3prl_upstream(S3PRLUpstream), []
+    for case_lens in S3PRL_UPSTREAM_LENS:
+        for normalize in (False, True):
+            ref.normalize = normalize
+            wavs = torch.zeros(len(case_lens), max(case_lens) + 37)  # the padded tensor may be wider than the longest
+            for i, n in enumerate(case_lens):
+                wavs[i, :n] = torch.randn(n, generator=g)
+            a_hs, a_len = ref(wavs, torch.tensor(case_lens))
+            b_hs, b_len = ref(wavs.unsqueeze(-1), torch.tensor(case_lens))
+            assert all(torch.equal(x, y) for x, y in zip(a_hs + a_len, b_hs + b_len))
+            cases.append({"lens": case_lens, "normalize": normalize, "hs": a_hs, "hs_len": a_len})
+    refused = []
+    for case_lens in S3PRL_UPSTREAM_REFUSED_LENS:
+        try:
+            ref(torch.zeros(len(case_lens), max(case_lens)), torch.tensor(case_lens))
+            refused.append(False)
+        except AssertionError:
+            refused.append(True)
+    torch.save({"inputs": {"hs": hs, "lens": lens}, "featurizer": featurizer,
+                "single_layer_has_weights": hasattr(single, "weights"),
+                "udm": {"hs": udm_hs.detach(), "hs_len": udm_len, "input_size": udm.input_size,
+                        "downsample_rate": udm.downsample_rate, "output_size": udm.output_size},
+                "s3prl_upstream": cases, "s3prl_upstream_refused": refused},
+               GOLDEN / "nn_upstream.pt")
+    print(f"nn: {len(featurizer)} featurizer cases, {len(cases)} S3PRLUpstream cases, refused {refused}")
+
+
+def make_hub_fixture():
+    """The entry names of the reference's s3prl.hub (s3prl/hub.py:40-54 options()), which the Runner resolves with
+    getattr(hub, name) and s3prl_b200.hub.install overrides."""
+    import json
+
+    import s3prl.hub as hub
+
+    names = sorted(hub.options())
+    (GOLDEN / "hub_entries.json").write_text(json.dumps(names, indent=0) + "\n")
+    print(f"hub: {len(names)} entries")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=None)
     args = ap.parse_args()
     GOLDEN.mkdir(parents=True, exist_ok=True)
+    activate()
     torch.manual_seed(0)
     if args.only in (None, "integer"):
         make_integer_fixture()
+    if args.only in (None, "nn"):
+        make_nn_fixture()
+    if args.only in (None, "hub"):
+        make_hub_fixture()
     if args.only in (None, "fbank"):
         make_fbank_fixture()
     if args.only in (None, "spectrogram"):

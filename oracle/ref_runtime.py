@@ -1,8 +1,9 @@
 """TEST INFRASTRUCTURE — run the reference itself (s3prl) on a fabricated checkpoint.
 
 Used by oracle/make_golden.py (fixtures) and by bench.py's `--impl reference` / cpu_baseline legs. The reference is
-found at /root/reference (build container) or oracle/_ref (the installed copy that travels to the GPU box, see
-oracle/build_ref.py). Nothing in the product package imports this module.
+the s3prl checkout beside this repository (../reference, or S3PRL_REFERENCE), else the copy installed under
+oracle/_ref (see oracle/build_ref.py).
+Nothing in the product package imports this module.
 """
 from __future__ import annotations
 
@@ -23,8 +24,10 @@ from s3prl_b200.upstream.convert import reference_model_cfg  # noqa: E402
 
 
 def reference_root() -> Optional[Path]:
-    for cand in (Path("/root/reference"), ROOT / "oracle" / "_ref"):
-        if (cand / "s3prl" / "upstream" / "hubert" / "expert.py").exists():
+    from build_ref import REFERENCE, TARGET, exists
+
+    for cand in (REFERENCE, TARGET):
+        if exists(cand / "s3prl" / "upstream" / "hubert" / "expert.py"):
             return cand
     return None
 
@@ -33,7 +36,7 @@ def activate() -> Path:
     """Put the reference on sys.path (once) and register the import shims it needs in this image."""
     root = reference_root()
     if root is None:
-        raise RuntimeError("the reference (s3prl) is neither at /root/reference nor installed under oracle/_ref")
+        raise RuntimeError("the reference (s3prl) is neither checked out at ../reference (or S3PRL_REFERENCE) nor installed under oracle/_ref")
     if str(root) not in sys.path:
         sys.path.insert(0, str(root))
     from s3prl_b200.run_downstream import install_shims

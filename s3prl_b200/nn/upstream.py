@@ -19,8 +19,8 @@ its definition rather than from the reference's code:
 
 ``Featurizer`` (``:234-349``) and ``UpstreamDownstreamModel`` (``:352-384``) are the reference's reduction and
 composition wrappers; the weighted layer sum runs in the fused CUDA kernel ``s3b_weighted_sum`` (+ its backward).
-Parity: ``tests/test_host_cpu.py::test_nn_featurizer_matches_reference_logic`` runs these classes next to the
-reference's own on the CPU; ``tests/test_api_gpu.py`` covers the device path.
+Parity: ``tests/test_host_cpu.py::test_nn_featurizer_matches_reference_logic`` checks these classes on the CPU
+against what the reference's own returned (tests/golden/nn_upstream.pt); ``tests/test_api_gpu.py`` covers the device path.
 """
 from __future__ import annotations
 

@@ -1,5 +1,6 @@
-"""CPU tests of the host-side logic: C-ABI symbol export, loud failure without a GPU, hub injection into the
-reference (when /root/reference is present), utterance sharding + gather over gloo with world_size 2."""
+"""CPU tests of the host-side logic: C-ABI symbol export, loud failure without a GPU, hub injection into s3prl.hub,
+the s3prl.nn mirrors against the reference's results (tests/golden), utterance sharding + gather over gloo with
+world_size 2."""
 import os
 import re
 import sys
@@ -9,7 +10,7 @@ import pytest
 import torch
 
 ROOT = Path(__file__).resolve().parents[1]
-REFERENCE = Path("/root/reference")
+GOLDEN = ROOT / "tests" / "golden"
 
 
 def test_cabi_exports_every_declared_symbol(s3b_lib):
@@ -117,27 +118,55 @@ def test_fabricated_state_dict_is_deterministic_and_loadable_layout():
     assert c["feature_extractor.conv_layers.3.0.bias"].shape == (512,)
 
 
-@pytest.mark.skipif(not REFERENCE.exists(), reason="reference tree not present (GPU box)")
-def test_hub_injection_into_reference():
-    """`getattr(s3prl.hub, name)` — what Runner._get_upstream does (runner.py:141) — yields our expert."""
+def test_hub_injection_into_reference(tmp_path):
+    """`getattr(s3prl.hub, name)` — what Runner._get_upstream does (runner.py:141) — yields our expert after
+    run_downstream.inject(), every other entry of the reference hub stays as it was, and the Featurizer the Runner
+    instantiates is ours. Runs against the reference's own s3prl when it is available (oracle/build_ref.py), else against
+    a stand-in package with the layout inject() touches and the reference hub's entry names (tests/golden/hub_entries.json,
+    recorded from the reference by oracle/make_golden.py)."""
+    import json
     import subprocess
 
+    names = json.loads((GOLDEN / "hub_entries.json").read_text())
+    assert {"hubert_base", "wavlm_base_plus", "fbank"} <= set(names)
+    reference = _reference_install()
+    if reference is None:
+        reference = tmp_path
+        pkg = tmp_path / "s3prl"
+        for sub in ("upstream", "downstream"):
+            (pkg / sub).mkdir(parents=True)
+            (pkg / sub / "__init__.py").write_text("")
+        (pkg / "__init__.py").write_text("")
+        (pkg / "hub.py").write_text("".join(f"def {n}(*args, **kwargs):\n    raise RuntimeError('stand-in')\n" for n in names))
+        (pkg / "upstream" / "interfaces.py").write_text("class Featurizer:\n    pass\n")
+        (pkg / "downstream" / "runner.py").write_text("from s3prl.upstream.interfaces import Featurizer\n\n\nclass Runner:\n    pass\n")
     code = (
+        "import json\n"
         "from s3prl_b200 import run_downstream as R\n"
-        "names = R.inject()\n"
+        "R.install_shims()\n"
         "import s3prl.hub as hub\n"
+        f"reference = json.loads(open({str(GOLDEN / 'hub_entries.json')!r}).read())\n"
+        "before = {n: getattr(hub, n) for n in reference}\n"
+        "names = R.inject()\n"
+        "from s3prl_b200 import hub as ours\n"
         "from s3prl_b200.upstream.expert import UpstreamExpert\n"
         "from s3prl_b200.upstream.baseline import FbankExpert\n"
+        "from s3prl_b200.upstream.featurizer import Featurizer\n"
         "e = getattr(hub, 'hubert_base')(ckpt=None, model_config=None, refresh=False)\n"
         "assert isinstance(e, UpstreamExpert) and e.get_downsample_rates('hidden_states') == 320\n"
         "assert isinstance(hub.fbank(), FbankExpert)\n"
         "assert isinstance(hub.wavlm_base_plus(), UpstreamExpert)\n"
+        "assert all(getattr(hub, n) is ours.ENTRIES[n] for n in reference if n in ours.ENTRIES)\n"
+        "assert all(getattr(hub, n) is before[n] for n in reference if n not in ours.ENTRIES)\n"
         "from s3prl.downstream.runner import Runner\n"
-        "print('OK', len(names))\n"
+        "import s3prl.downstream.runner as runner, s3prl.upstream.interfaces as interfaces\n"
+        "assert runner.Featurizer is Featurizer and interfaces.Featurizer is Featurizer\n"
+        "print('OK', len(names), hub.__file__)\n"
     )
-    env = dict(os.environ, PYTHONPATH=f"{REFERENCE}:{ROOT}")
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
+    env = dict(os.environ, PYTHONPATH=f"{reference}:{ROOT}")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=str(tmp_path), timeout=600)
     assert r.returncode == 0 and "OK" in r.stdout, r.stderr[-2000:]
+    print(r.stdout.strip())
 
 
 def test_product_never_imports_the_oracle():
@@ -354,18 +383,17 @@ def test_huggingface_second_oracle(kind, kw):
         assert ((a - b).norm() / b.norm()).item() < 5e-6
 
 
-@pytest.mark.skipif(not (REFERENCE / "s3prl" / "nn" / "upstream.py").exists() and not (ROOT / "oracle" / "_ref" / "s3prl").exists(),
-                    reason="needs the reference (s3prl.nn) to compare against")
+def _nn_golden():
+    """What the reference's s3prl.nn classes returned on the inputs below (oracle/make_golden.py make_nn_fixture)."""
+    return torch.load(GOLDEN / "nn_upstream.pt", weights_only=False)
+
+
 def test_nn_featurizer_matches_reference_logic(monkeypatch):
     """s3prl_b200.nn.Featurizer / UpstreamDownstreamModel against the reference's own classes (s3prl/nn/upstream.py:234-384)
     on the CPU: layer selection, normalize, single-layer pass-through, weights and their gradient. The fused CUDA sum is
     replaced by its torch definition for this host-logic test (the kernel itself is pinned in tests/test_api_gpu.py)."""
     sys.path.insert(0, str(ROOT / "oracle"))
-    import ref_runtime
-
-    ref_runtime.activate()
-    from s3prl.nn.upstream import Featurizer as RefFeaturizer
-    from s3prl.nn.upstream import UpstreamDownstreamModel as RefUDM
+    from make_golden import FakeUpstream
 
     import s3prl_b200.upstream.featurizer as fused
     from s3prl_b200.nn import Featurizer, UpstreamDownstreamModel
@@ -377,26 +405,22 @@ def test_nn_featurizer_matches_reference_logic(monkeypatch):
         fused.weighted_sum([torch.zeros(1, 4, 8)] * 2, torch.ones(2) / 2)
     monkeypatch.setattr(fused, "weighted_sum", torch_sum)
 
-    class FakeUpstream:
-        def __init__(self, n):
-            self.num_layers, self.hidden_sizes, self.downsample_rates = n, [16] * n, [320] * n
-
-    g = torch.Generator().manual_seed(0)
-    hs = [torch.randn(3, 7, 16, generator=g) for _ in range(5)]
-    lens = [torch.tensor([7, 5, 2])] * 5
-    for sel, norm in ((None, False), ([4, 0, 2], False), (None, True), ([1, 3], True)):
-        ours, ref = Featurizer(FakeUpstream(5), sel, norm), RefFeaturizer(FakeUpstream(5), sel, norm)
-        w = torch.randn(len(ours.weights), generator=g)
+    fx = _nn_golden()
+    hs, lens = fx["inputs"]["hs"], fx["inputs"]["lens"]
+    cases = ((None, False), ([4, 0, 2], False), (None, True), ([1, 3], True))
+    assert len(fx["featurizer"]) == len(cases)
+    for (sel, norm), ref in zip(cases, fx["featurizer"]):
+        ours = Featurizer(FakeUpstream(5), sel, norm)
         with torch.no_grad():
-            ours.weights.copy_(w), ref.weights.copy_(w)
-        assert ours.layer_selections == ref.layer_selections
-        (a, al), (b, bl) = ours(hs, lens), ref(hs, lens)
-        assert torch.allclose(a, b, atol=1e-6) and torch.equal(al, bl)
-        a.square().sum().backward(), b.square().sum().backward()
-        assert torch.allclose(ours.weights.grad, ref.weights.grad, rtol=1e-5, atol=1e-6)
-        assert ours.output_size == ref.output_size == 16 and ours.downsample_rate == ref.downsample_rate == 320
-    one, one_ref = Featurizer(FakeUpstream(1)), RefFeaturizer(FakeUpstream(1))
-    assert not hasattr(one, "weights") and not hasattr(one_ref, "weights")
+            ours.weights.copy_(ref["weights"])
+        assert ours.layer_selections == ref["layer_selections"]
+        a, al = ours(hs, lens)
+        assert torch.allclose(a, ref["hs"], atol=1e-6) and torch.equal(al, ref["hs_len"])
+        a.square().sum().backward()
+        assert torch.allclose(ours.weights.grad, ref["grad"], rtol=1e-5, atol=1e-6)
+        assert ours.output_size == ref["output_size"] == 16 and ours.downsample_rate == ref["downsample_rate"] == 320
+    one = Featurizer(FakeUpstream(1))
+    assert not hasattr(one, "weights") and not fx["single_layer_has_weights"]
     assert one(hs[:1], lens[:1])[0] is hs[0]
 
     class Up(torch.nn.Module):
@@ -405,72 +429,54 @@ def test_nn_featurizer_matches_reference_logic(monkeypatch):
         def forward(self, wav, wav_len):
             return hs, lens
 
-    class Down(torch.nn.Module):
+    class Down(torch.nn.Module):  # no reduction: the stored result is exact on any CPU
         output_size = 3
 
         def forward(self, h, h_len, scale=1.0):
-            return h.mean(-1) * scale, h_len
+            return h[..., :3] * scale, h_len
 
     f = Featurizer(Up())
-    ours, ref = UpstreamDownstreamModel(Up(), f, Down()), RefUDM(Up(), f, Down())
-    (a, al), (b, bl) = ours(None, None, scale=2.0), ref(None, None, scale=2.0)
-    assert torch.equal(a, b) and torch.equal(al, bl)
-    assert (ours.input_size, ours.downsample_rate, ours.output_size) == (ref.input_size, ref.downsample_rate, ref.output_size)
+    ours, ref = UpstreamDownstreamModel(Up(), f, Down()), fx["udm"]
+    a, al = ours(None, None, scale=2.0)
+    assert torch.equal(a, ref["hs"]) and torch.equal(al, ref["hs_len"])
+    assert (ours.input_size, ours.downsample_rate, ours.output_size) == (ref["input_size"], ref["downsample_rate"], ref["output_size"])
     with pytest.raises(NotImplementedError):
         UpstreamDownstreamModel(Up(), f, Down(), upstream_trainable=True)
 
 
-def _fake_wrapped(cls, ours: bool):
-    """An S3PRLUpstream (ours or the reference's) around a fake three-layer upstream with the conv stack's frame rule."""
-
-    class Fake(torch.nn.Module):
-        def forward(self, wavs):
-            frames = max((len(w) - 400) // 320 + 1 if len(w) >= 400 else 0 for w in wavs)
-            base = torch.arange(len(wavs) * frames * 2, dtype=torch.float32).view(len(wavs), frames, 2)
-            return {"hidden_states": [base + k for k in range(3)]}
-
-    obj = cls.__new__(cls)
-    torch.nn.Module.__init__(obj)
-    obj.upstream, obj.normalize = Fake(), False
-    obj._hidden_sizes, obj._downsample_rates = [2] * 3, [320] * 3
-    if not ours:
-        obj._num_layers = 3
-    return obj
-
-
-@pytest.mark.skipif(not (REFERENCE / "s3prl" / "nn" / "upstream.py").exists() and not (ROOT / "oracle" / "_ref" / "s3prl").exists(),
-                    reason="needs the reference (s3prl.nn) to compare against")
 def test_s3prl_upstream_bookkeeping_matches_reference_class():
     """The length bookkeeping of s3prl_b200.nn.S3PRLUpstream.forward (frame count per layer, last-frame repeat / cut,
-    h_len, the 0.05 s minimum, normalize) next to the reference's own class (s3prl/nn/upstream.py:166-231) on the same
-    fake upstream: identical tensors, and the same AssertionError where the reference refuses a 2x frame mismatch."""
+    h_len, the 0.05 s minimum, normalize) against what the reference's own class (s3prl/nn/upstream.py:166-231) returned
+    on the same fake upstream: identical tensors, and an AssertionError where the reference refuses a 2x frame mismatch."""
     sys.path.insert(0, str(ROOT / "oracle"))
-    import ref_runtime
-
-    ref_runtime.activate()
-    from s3prl.nn.upstream import S3PRLUpstream as Ref
+    from make_golden import fake_s3prl_upstream
 
     from s3prl_b200.nn import S3PRLUpstream as Ours
 
-    ref, ours = _fake_wrapped(Ref, False), _fake_wrapped(Ours, True)
+    fx = _nn_golden()
+    ours = fake_s3prl_upstream(Ours)
+    # the fake upstream reads only the lengths, so these waveforms need not be the ones the reference was given
     g = torch.Generator().manual_seed(0)
-    for lens in ([16000, 9000, 3200], [16001, 480], [700, 500], [32000, 31999], [1281, 1280, 1279], [48000]):
-        for normalize in (False, True):
-            ref.normalize = ours.normalize = normalize
-            width = max(lens) + 37  # the padded tensor may be wider than the longest utterance
-            wavs = torch.zeros(len(lens), width)
-            for i, n in enumerate(lens):
-                wavs[i, :n] = torch.randn(n, generator=g)
-            for w in (wavs, wavs.unsqueeze(-1)):
-                (a_hs, a_len), (b_hs, b_len) = ref(w, torch.tensor(lens)), ours(w, torch.tensor(lens))
-                assert len(a_hs) == len(b_hs) == 3
-                assert all(torch.equal(x, y) for x, y in zip(a_hs, b_hs)), lens
-                assert all(torch.equal(x, y) for x, y in zip(a_len, b_len)), lens
-    for lens in ([960, 961], [1000, 900]):  # 2 frames from the conv rule where ceil(L / 320) = 4: refused by both
-        wavs = torch.zeros(len(lens), max(lens))
-        for cls_obj in (ref, ours):
-            with pytest.raises(AssertionError):
-                cls_obj(wavs, torch.tensor(lens))
+    cases = [(lens, normalize) for lens in ([16000, 9000, 3200], [16001, 480], [700, 500], [32000, 31999],
+                                            [1281, 1280, 1279], [48000]) for normalize in (False, True)]
+    assert [(c["lens"], c["normalize"]) for c in fx["s3prl_upstream"]] == cases
+    for ref in fx["s3prl_upstream"]:
+        lens = ref["lens"]
+        ours.normalize = ref["normalize"]
+        width = max(lens) + 37  # the padded tensor may be wider than the longest utterance
+        wavs = torch.zeros(len(lens), width)
+        for i, n in enumerate(lens):
+            wavs[i, :n] = torch.randn(n, generator=g)
+        for w in (wavs, wavs.unsqueeze(-1)):
+            b_hs, b_len = ours(w, torch.tensor(lens))
+            assert len(ref["hs"]) == len(b_hs) == 3
+            assert all(torch.equal(x, y) for x, y in zip(ref["hs"], b_hs)), lens
+            assert all(torch.equal(x, y) for x, y in zip(ref["hs_len"], b_len)), lens
+    # 2 frames from the conv rule where ceil(L / 320) = 4: refused by the reference, and here
+    assert fx["s3prl_upstream_refused"] == [True, True]
+    for lens in ([960, 961], [1000, 900]):
+        with pytest.raises(AssertionError):
+            ours(torch.zeros(len(lens), max(lens)), torch.tensor(lens))
 
 
 def test_s3prl_upstream_wrapper_layer_counts():
@@ -485,13 +491,16 @@ def test_s3prl_upstream_wrapper_layer_counts():
 
 
 def _reference_install():
-    for cand in (REFERENCE, ROOT / "oracle" / "_ref"):
-        if (cand / "s3prl" / "downstream" / "runner.py").exists():
-            return cand
-    return None
+    """The s3prl checkout beside the repository (or S3PRL_REFERENCE), else the install under oracle/_ref that build()
+    makes from it (oracle/build_ref.py), else None."""
+    sys.path.insert(0, str(ROOT / "oracle"))
+    import ref_runtime
+
+    return ref_runtime.reference_root()
 
 
-@pytest.mark.skipif(_reference_install() is None, reason="reference neither at /root/reference nor installed in oracle/_ref")
+# This test runs the reference's own training loop, so no stored result can stand in for the reference here.
+@pytest.mark.skipif(_reference_install() is None, reason="needs the reference (s3prl): check it out at ../reference (or set S3PRL_REFERENCE) before build()")
 def test_launcher_runs_reference_runner_on_synthetic_librispeech(tmp_path):
     """BASELINE config 5 plumbing without a GPU: the launcher's synthetic LibriSpeech-shaped dataloader
     (s3prl_b200/synthetic.py, replacing ctc/data.py:73-86 load_dataset) drives the reference's UNMODIFIED Runner.train
